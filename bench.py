@@ -39,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from as it found it
 for p in (os.path.join(ROOT, "4d-gaussian-splatting_b200"), os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
@@ -223,6 +224,8 @@ class Runner:
         self.res_ready = torch.cuda.Event()
         self.pending = False
         self.last = None
+        self.keep_outputs = False      # --dump-outputs: hold the last view's rasterizer outputs (self.outputs())
+        self.last_out = None
         # the exchange (and the factor path that avoids V dense dL_dsh accumulations) whenever a step has > 1 view
         self.exchange = impl == "ours" and self.backward and (world > 1 or len(wl.view_ids) > 1) and \
             os.environ.get("FDGS_DENSE_ALLREDUCE") is None
@@ -286,6 +289,8 @@ class Runner:
                         self.g_ready[i][b] = None
                 if self.backward:
                     (color, radii, depth, alpha, flow, covs), means2D = self._raster(st)
+                    if self.keep_outputs:
+                        self.last_out = dict(color=color, radii=radii, depth=depth, alpha=alpha, flow=flow, covs=covs)
                     if host_inputs:
                         cur.wait_event(ready)
                     loss = (color * G).sum() / self.views_total
@@ -306,6 +311,8 @@ class Runner:
                 else:
                     with torch.no_grad():
                         (color, radii, depth, alpha, flow, covs), means2D = self._raster(st)
+                    if self.keep_outputs:
+                        self.last_out = dict(color=color, radii=radii, depth=depth, alpha=alpha, flow=flow, covs=covs)
                     result = color.mean() if result is None else result + color.mean()
                     self.last = (result, radii, means2D)
         finally:
@@ -350,6 +357,18 @@ class Runner:
         self.pending = False
         return float(self.res_host[0])
 
+    def outputs(self):
+        """What the last step handed its caller: the rasterizer outputs of the last view and the loss; with a backward
+        also the gradients of the Gaussian parameters and of the screen-space means (summed over the step's views)."""
+        out = dict(self.last_out, loss=self.last[0])
+        # covariance rows of Gaussians the preprocess culled (radii 0) are never written, as in the reference: zero them
+        # so that two runs or builds compare equal
+        out["covs"] = torch.where((out["radii"] > 0)[:, None], out["covs"], 0.0)
+        if self.backward:
+            out.update({"grad_" + k: v.grad for k, v in self.wl.params.items()})
+            out["grad_means2D"] = self.last[2].grad
+        return out
+
     def h2d_bytes(self):
         cam = sum(h.numel() * 4 for c in self.wl.cam_host for h in c.values())
         img = sum(g.numel() * 4 for g in self.wl.G_host) if self.backward else 0
@@ -382,6 +401,31 @@ def timed(fn, steps, warmup, device, world, finish=None):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     return ms / steps, wall / steps * 1e3
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, outputs, P):
+    """--dump-outputs: one float32 DIR/<name>.npy per output.  When everything would exceed DUMP_BYTES, the per-Gaussian
+    arrays (first dimension P) keep the same seeded sample of rows -- the largest power of two that fits -- whose
+    indices go to DIR/gaussian_index.npy (float64), so that two builds can be compared output for output."""
+    outputs = {k: v.detach() for k, v in outputs.items() if v is not None}
+    per_gaussian = [k for k, v in outputs.items() if v.dim() > 0 and v.shape[0] == P]
+    fixed = sum(4 * v.numel() for k, v in outputs.items() if k not in per_gaussian)
+    row = sum(4 * outputs[k][0].numel() for k in per_gaussian)
+    index = None
+    if fixed + P * row > DUMP_BYTES:
+        n = 1 << int(math.log2(max((DUMP_BYTES - fixed) // (row + 8), 1)))
+        g = torch.Generator().manual_seed(0)
+        index = torch.sort(torch.randperm(P, generator=g)[:n]).values
+    os.makedirs(path, exist_ok=True)
+    for k, v in outputs.items():
+        if index is not None and k in per_gaussian:
+            v = v[index.to(v.device)]
+        np.save(os.path.join(path, k + ".npy"), v.float().cpu().numpy())
+    if index is not None:
+        np.save(os.path.join(path, "gaussian_index.npy"), index.double().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -536,6 +580,8 @@ def run_train(args, rank, device):
     sampler.start()
     ms, wall = timed(one, args.steps, args.warmup, device, 1)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict({"param_" + k: v for k, v in raw.items()}, loss=losses[-1]), P)
     curve = [float(x) for x in torch.stack(losses).cpu()]
     return {"metric": WORKLOADS["cfg4"]["metric"], "value": 1e3 / ms, "unit": "it/s", "n_gpus": 1, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -605,6 +651,8 @@ def run_train_step(args, rank, device):
     sampler.start()
     ms, wall = timed(step, args.steps, args.warmup, device, 1)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict({"param_" + k: v for k, v in lv.items()}, loss=last[0]), cfg["P"])
     mpix = cfg["W"] * cfg["H"] / 1e6
     # phase breakdown (CUDA events around the phases of a few extra steps)
     phases = {}
@@ -649,7 +697,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--rigid", action="store_true", help="cfg4: lambda_rigid = 1.0 (kNN rigidity loss) like configs/dnerf/lego.yaml")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     spec = WORKLOADS[args.workload]
 
@@ -706,6 +758,7 @@ def main():
         assert len(view_ids) > 0, "more ranks than views"
     wl = Workload(args.workload, device, view_ids)
     runner = Runner(wl, "ours" if args.impl == "ours" else "ref", eff_world, views_total)
+    runner.keep_outputs = bool(args.dump_outputs) and rank == 0
     mpix = wl.W * wl.H / 1e6
 
     # ---- value: resident inputs -------------------------------------------------------------------
@@ -716,6 +769,9 @@ def main():
     sampler.start()
     ms_step, wall_ms = timed(lambda: runner.step(False), args.steps, args.warmup, device, eff_world)
     clocks = sampler.stop()
+    if runner.keep_outputs:
+        dump_outputs(args.dump_outputs, runner.outputs(), wl.P)
+        runner.keep_outputs, runner.last_out = False, None
     launches = (fdgs.launch_count() - launches0) if args.impl == "ours" else None
     value = views_total * mpix / (ms_step * 1e-3)
 

@@ -1,6 +1,7 @@
 """Shared helpers of the parity tests: seeded configurations, runners for the three
 implementations (CUDA path through the extension, CPU oracle, compiled reference) and the
 comparison metrics (SURVEY.md section 8d)."""
+import hashlib
 import os
 
 import numpy as np
@@ -155,6 +156,100 @@ def psnr(a, b):
 def golden(name):
     path = os.path.join(GOLDEN_DIR, "golden_%s.npz" % name)
     return np.load(path) if os.path.exists(path) else None
+
+
+# ---- compact records of the reference at sizes too large to store whole (tests/golden/ref_*.npz, written by
+# tools/ref_golden.py from the compiled reference).  Bit-exact outputs are kept as SHA-256 digests; gradients as the
+# mean of the reference's reruns on a seeded sample of rows (the largest rows plus random ones) with the reference's
+# run-to-run spread on that sample and over the whole tensor, and the norm of the whole mean tensor.
+SAMPLE_TOP, SAMPLE_RANDOM, SAMPLE_COLS = 16, 32, 12
+GRAD_STATS = ("nm_full", "l2n_full", "l2max_full", "l2n", "l2max", "mxn", "rmed")
+GRAD_EMPTY, GRAD_ZERO = -1.0, 0.0          # one-element records: the reference returned an empty / an all-zero tensor
+
+
+def ref_record(name):
+    """tests/golden/ref_<name>.npz as a dict: every digest by its name (a str), every other array as stored."""
+    with np.load(os.path.join(GOLDEN_DIR, "ref_%s.npz" % name)) as z:
+        rec = {k: z[k] for k in z.files if k != "digests"}
+        rec.update(s.decode().split("=", 1) for s in z["digests"])
+    return rec
+
+
+def pack_digests(d):
+    return np.array(["%s=%s" % kv for kv in d.items()], dtype="S")
+
+
+def digest(t):
+    """SHA-256 of a tensor's values: floats by their fp32 bit patterns, integers widened to int64."""
+    a = np.ascontiguousarray(to_np(t) if hasattr(t, "detach") else np.asarray(t))
+    if a.dtype.kind == "f":
+        assert a.dtype == np.float32, a.dtype
+    else:
+        a = a.astype(np.int64)
+    return "%s:%s" % (a.size, hashlib.sha256(a.reshape(-1).tobytes()).hexdigest())
+
+
+def list_digests(lists):
+    """Digests of the tile lists of check_tile_lists's dict layout."""
+    return dict(point_list=digest(np.asarray(lists["point_list"]).reshape(-1)),
+                ranges=digest(np.asarray(lists["ranges"]).reshape(-1, 2)),
+                n_contrib=digest(np.asarray(lists["n_contrib"]).reshape(-1)), num_rendered=str(int(lists["num_rendered"])))
+
+
+def median_row_err(x, m):
+    d = (x - m).norm(dim=1)
+    n = m.norm(dim=1)
+    keep = n > 0
+    return (d[keep] / n[keep]).median().item() if bool(keep.any()) else 0.0
+
+
+def pack_grad(rows, cols, mean, stats):
+    """One float32 array: [len(rows), len(cols), GRAD_STATS..., rows, cols, mean (rows x cols)]; indices < 2^24."""
+    assert len(rows) == 0 or int(np.max(rows)) < (1 << 24)
+    return np.concatenate([[len(rows), len(cols)], stats, rows, cols, np.asarray(mean).reshape(-1)]).astype(np.float32)
+
+
+def grad_record(runs, seed):
+    """Record of K reference reruns of one gradient tensor (list of K tensors [P, ...]) for grad_sample."""
+    if runs[0].numel() == 0:
+        return np.array([GRAD_EMPTY], np.float32)
+    P = runs[0].shape[0]
+    flat = lambda r: r.detach().reshape(P, -1).double()
+    m = sum(flat(r) for r in runs) / len(runs)
+    nm = m.norm().item()
+    if nm == 0.0:
+        return np.array([GRAD_ZERO], np.float32)
+    rel = [(flat(r) - m).norm().item() / nm for r in runs]
+    n = m.norm(dim=1)
+    nz = torch.nonzero(n > 0).squeeze(1)
+    g = torch.Generator().manual_seed(seed)
+    pick = torch.randperm(nz.numel(), generator=g)[:SAMPLE_RANDOM].to(nz.device)
+    rows = torch.unique(torch.cat([torch.topk(n, min(SAMPLE_TOP, nz.numel())).indices, nz[pick]]))
+    live = torch.nonzero(m.abs().amax(0) > 0).squeeze(1)
+    cols = live[torch.sort(torch.randperm(live.numel(), generator=g)[:SAMPLE_COLS]).values.to(live.device)]
+    S = torch.stack([flat(r)[rows][:, cols] for r in runs]).cpu()
+    rows, cols = rows.cpu(), cols.cpu()
+    del m, n
+    ms = S.mean(0)
+    nms, scs = ms.norm().item(), ms.abs().max().item()
+    rels = [(s - ms).norm().item() / nms for s in S]
+    stats = [nm, float(np.sqrt(np.mean(np.square(rel)))), max(rel), float(np.sqrt(np.mean(np.square(rels)))), max(rels),
+             max((s - ms).abs().max().item() for s in S) / scs, max(median_row_err(s, ms) for s in S)]
+    return pack_grad(rows.numpy(), cols.numpy(), ms.numpy(), stats)
+
+
+def grad_sample(p, a):
+    """p: a grad_record (neither GRAD_EMPTY nor GRAD_ZERO); a: our gradient tensor.  Returns (ours on the record's
+    sample, the reference mean there, | |ours| / |reference mean| - 1 | over the whole tensor, the statistics by name)."""
+    nr, nc = int(p[0]), int(p[1])
+    st = dict(zip(GRAD_STATS, p[2:2 + len(GRAD_STATS)].astype(np.float64).tolist()))
+    o = 2 + len(GRAD_STATS)
+    rows = torch.from_numpy(p[o:o + nr].astype(np.int64))
+    cols = torch.from_numpy(p[o + nr:o + nr + nc].astype(np.int64))
+    mean = torch.from_numpy(p[o + nr + nc:].astype(np.float64)).reshape(nr, nc)
+    a = a.detach().double().reshape(a.shape[0], -1)
+    s = a[rows.to(a.device)][:, cols.to(a.device)].cpu()
+    return s, mean, abs(a.norm().item() / st["nm_full"] - 1.0), st
 
 
 def to_np(t):

@@ -54,35 +54,26 @@ def test_fused_prologue_matches_getter_path(name, aux):
 def test_raw_entry_vs_reference_render_at_cfg3():
     """VERDICT r1 next #4: gradients w.r.t. the RAW parameters against the reference rasterizer under the reference's
     own torch prologue (getters + autograd), at cfg3.  Blend-level / SH / position tensors to 1e-4; the covariance chain
-    against the reference's own run-to-run spread (it is not reproducible to 1e-4 at this size)."""
-    import oracle_py
-    if not oracle_py.ref_available():
-        pytest.skip("oracle/_ref/ref_rasterizer.so not present")
-    import ref_api
+    against the reference's own run-to-run spread (it is not reproducible to 1e-4 at this size).  The reference's three
+    runs are a record (tests/golden/ref_raw_cfg3.npz, tools/ref_golden.py): a pixel sample of its image, and per leaf
+    the mean gradient on a sample of rows with the runs' spread there and over the whole tensor."""
+    rec = helpers.ref_record("raw_cfg3")
     cfg, cam, sc, st = helpers.build("cfg3", device=DEV)
     cam = cam.to(DEV)
     g = torch.Generator().manual_seed(77)
     G = torch.randn(3, cfg["H"], cfg["W"], generator=g).to(DEV)
-
-    def ref_run():
-        R = RawModel(sc, seed=2, requires_grad=True)
-        m2 = torch.zeros_like(R._xyz, requires_grad=True)
-        out = ref_api.rasterize(st, R.get_xyz, m2, R.get_opacity, R.get_features, torch.zeros(sc.P, 2, device=DEV), R.get_t,
-                                R.get_scaling, R.get_scaling_t, R.get_rotation, R.get_rotation_r)
-        (out[0] * G).sum().backward()
-        return R, out[0].detach()
-
-    runs = [ref_run() for _ in range(3)]
     B = RawModel(sc, seed=2, requires_grad=True)
     pb = _render_and_backward(B, cam, Pipe(), G)
-    assert helpers.psnr(helpers.to_np(pb["render"]), helpers.to_np(runs[0][1])) > 90.0
+    pix = torch.from_numpy(rec["pixels"]).long().to(DEV)
+    assert helpers.psnr(helpers.to_np(pb["render"].reshape(3, -1)[:, pix]), rec["image"]) > 90.0
     for k, b in B.leaves().items():
-        rs = [r[0].leaves()[k].grad for r in runs]
-        m = torch.stack([x.double() for x in rs]).mean(0)
-        nm = m.norm().item()
-        l2 = ((b.grad.double() - m).norm() / nm).item()
-        spread = max(((x.double() - m).norm() / nm).item() for x in rs)
+        s, m, norm_dev, st = helpers.grad_sample(rec[k], b.grad)
+        l2 = ((s - m).norm() / m.norm()).item()
+        # the runs' spread over the whole tensor or on the sample, whichever is larger: on the covariance chain a few
+        # noisy rows outside the sample carry most of the whole tensor's spread
+        spread = max(st["l2max"], st["l2max_full"])
         assert l2 < max(1e-4, 4 * spread), (k, l2, spread)
+        assert norm_dev < max(1e-4, 4 * st["l2max_full"]), (k, "norm", norm_dev, st["l2max_full"])
         print("raw grad %-13s vs reference render(): l2 %.2e (reference spread %.2e)" % (k, l2, spread))
 
 

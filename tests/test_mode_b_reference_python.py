@@ -1,38 +1,37 @@
-"""CPU (this container only): INTEGRATION.md mode B -- the reference's OWN gaussian_renderer/diff_gaussian_rasterization.py
-(classes and autograd function, lines after its JIT-load preamble) executed with `_C` bound to this repo's extension.
-The reference tree exists only here (never on the GPU box), so the test is skipped when it is absent, and without a
-GPU it can only go as far as the extension's first device check: that point is reached only if pybind accepted all
-30 positional arguments in the reference's order and types (a signature mismatch raises TypeError first)."""
+"""CPU: INTEGRATION.md mode B -- the reference's OWN gaussian_renderer/diff_gaussian_rasterization.py (classes and
+autograd function, lines after its JIT-load preamble) driving this repo's extension as its `_C`.  What that layer
+passes is recorded in tests/golden/ref_python_call.json (tools/ref_golden.py --python-call ran it with a recording
+`_C`): the settings' field names and the 30 positional arguments of `_C.rasterize_gaussians` in the reference's order
+and types.  The test replays that call on the extension; without a GPU it can only go as far as the extension's first
+device check, and that point is reached only if pybind accepted the reference's argument list (a signature mismatch
+raises TypeError first)."""
+import json
 import os
 
 import pytest
-import torch
 
 import helpers
 
-REF_FILE = "/root/reference/gaussian_renderer/diff_gaussian_rasterization.py"
 
-
-@pytest.mark.skipif(not os.path.exists(REF_FILE), reason="reference tree not present")
 def test_reference_python_layer_binds_to_our_extension():
     import fdgs
-    src = open(REF_FILE).read()
-    start = src.index("def cpu_deep_copy_tuple")       # everything after the reference's `_C = load(...)` JIT preamble
-    ns = {"torch": torch, "nn": torch.nn, "_C": fdgs.ext(), "__name__": "ref_dgr_on_fdgs"}
-    from typing import NamedTuple
-    ns["NamedTuple"] = NamedTuple
-    exec(compile(src[start:], REF_FILE, "exec"), ns)
     from gaussian_renderer import GaussianRasterizationSettings as Ours
-    assert ns["GaussianRasterizationSettings"]._fields == Ours._fields
+    with open(os.path.join(helpers.GOLDEN_DIR, "ref_python_call.json")) as f:
+        rec = json.load(f)
+    assert list(Ours._fields) == rec["fields"]
     cfg, cam, sc, st = helpers.build("tiny")
-    rast = ns["GaussianRasterizer"](ns["GaussianRasterizationSettings"](**st))
-    m2 = torch.zeros_like(sc.means3D)
-    # the reference's own validation messages come from the reference's own code
-    with pytest.raises(Exception, match="excatly one of either SHs or precomputed colors"):
-        rast(sc.means3D, m2, sc.opacities, scales=sc.scales, rotations=sc.rotations)
-    # full call: reference Python -> _C.rasterize_gaussians(30 positional args) -> our shim.  On CPU tensors our shim
-    # stops at its device check -- after pybind matched the reference's argument list.
+    import torch
+    inputs = dict(means3D=sc.means3D, opacities=sc.opacities, shs=sc.shs, flow_2d=sc.flow_2d, ts=sc.ts, scales=sc.scales,
+                  scales_t=sc.scales_t, rotations=sc.rotations, rotations_r=sc.rotations_r, empty=torch.Tensor([]))
+    inputs.update({"settings." + k: v for k, v in st.items()})
+    casts = {"float": float, "int": int, "bool": bool}
+    args = []
+    for a in rec["rasterize_gaussians"]:
+        (kind, v), = a.items()
+        args.append(inputs[v] if kind == "tensor" else casts[kind](v))
+    assert len(args) == 30
+    # full call: the reference's argument list -> our shim.  On CPU tensors our shim stops at its device check -- after
+    # pybind matched the reference's argument list.
     with pytest.raises(RuntimeError, match="means3D must be a CUDA tensor"):
-        rast(means3D=sc.means3D, means2D=m2, opacities=sc.opacities, shs=sc.shs, flow_2d=sc.flow_2d, ts=sc.ts, scales=sc.scales,
-             scales_t=sc.scales_t, rotations=sc.rotations, rotations_r=sc.rotations_r)
+        fdgs.ext().rasterize_gaussians(*args)
     assert hasattr(fdgs.ext(), "rasterize_gaussians_backward") and hasattr(fdgs.ext(), "mark_visible")
